@@ -4,6 +4,7 @@
   python bench.py --gpus 1 --steps 20 --warmup 3            # this repo's CUDA path
   python bench.py --impl reference --steps 3 --warmup 1     # the reference's CPU algorithm (oracle port)
   torchrun ... bench.py --gpus N ...                        # one rank per GPU
+  python bench.py ... --dump-outputs bench_outputs          # also write the last timed build's result as .npy files
 
 A "step" is one complete two-layer build (rmi_lib::train) of the workload
 `linear,linear 1048576 on 200M synthetic uint64` (BASELINE.json configs[1]) per GPU:
@@ -57,7 +58,48 @@ def parse_args():
     ap.add_argument("--no-extras", action="store_true", help="skip extra_configs")
     ap.add_argument("--e2e-steps", type=int, default=5)
     ap.add_argument("--extra-steps", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the result of the last timed build to DIR/<name>.npy (see dump_outputs)")
     return ap.parse_args()
+
+
+DUMP_BYTES = 64_000_000
+
+
+def result_arrays(r) -> dict:
+    """What a caller of the timed build receives (a TrainedRMI, or the oracle's OracleRMI for --impl reference),
+    copied out of the library's result memory so that later builds cannot overwrite it."""
+    if hasattr(r, "l0"):
+        r = {"model_max_error": r.max_error, "model_max_error_idx": r.max_error_idx, "model_avg_error": r.avg_error,
+             "model_avg_l2_error": r.avg_l2_error, "model_avg_log2_error": r.avg_log2_error,
+             "model_max_log2_error": r.max_log2_error, "l0_fparams": r.l0.fp, "l0_iparams": r.l0.ip,
+             "l0_table32": r.l0.t32, "l0_radix_index": r.l0.a1, "l0_pivots": r.l0.a2, "l1_params": r.l1_params,
+             "last_layer_max_l1s": r.l1_errors}
+    else:
+        r = vars(r)
+    import numpy as np
+    out = {"stats": np.array([r[k] for k in ("model_max_error", "model_max_error_idx", "model_avg_error", "model_avg_l2_error",
+                                             "model_avg_log2_error", "model_max_log2_error")], dtype=np.float64)}
+    for k in ("l0_fparams", "l0_iparams", "l0_table32", "l0_radix_index", "l0_pivots", "l1_params", "last_layer_max_l1s"):
+        if r[k] is not None and len(r[k]):
+            out[k] = np.array(r[k], dtype=np.float64)
+    return out
+
+
+def dump_outputs(arrays: dict, d: str) -> None:
+    """DIR/<name>.npy for every array of result_arrays, float64 (integers are exact below 2^53).  stats holds
+    max_error, max_error_idx, avg_error, avg_l2_error, avg_log2_error, max_log2_error.  Arrays of more than 1 MB
+    share what is left of DUMP_BYTES: past it, each keeps the same fixed rows (numpy default_rng(0), sorted)
+    as every other array of its length, so that the leaf parameters and error bounds still describe the same leaves."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    big = {k for k, a in arrays.items() if a.nbytes > 1 << 20}
+    room = DUMP_BYTES - sum(a.nbytes + 4096 for k, a in arrays.items() if k not in big) - 4096 * len(big)
+    frac = min(1.0, room / max(1, sum(arrays[k].nbytes for k in big)))
+    for k, a in arrays.items():
+        if k in big and frac < 1.0:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], int(a.shape[0] * frac), replace=False))]
+        np.save(os.path.join(d, k + ".npy"), a)
 
 
 def workload_config(args, world):
@@ -232,7 +274,10 @@ def run_reference(args, rank, world):
         time_oracle(keys, args.spec, args.leaves)
     t = []
     for _ in range(args.steps):
-        t.append(time_oracle(keys, args.spec, args.leaves)[0])
+        dt, r = time_oracle(keys, args.spec, args.leaves)
+        t.append(dt)
+    if args.dump_outputs:
+        dump_outputs(result_arrays(r), args.dump_outputs)
     tot = sum(t)
     val = n * args.steps / tot
     sample = (f"every step = one build of {n} uniform uint64 keys (numpy MT19937(42), sorted), {args.spec} {args.leaves}: "
@@ -385,6 +430,8 @@ def main():
     if rank == 0:
         clocks.sample_now()
     launches = rmi_b200.kernel_launch_count() - launches0
+    # written at the end, outside every timed region; copied now, before a later build can reuse the result's memory
+    outputs = result_arrays(res) if args.dump_outputs and rank == 0 else None
     phase_ms = phase_ms / 1e6
     value = (n * world) / (ms_per_step / 1e3)
 
@@ -596,6 +643,8 @@ def main():
            "roofline": roofline, "cpu_baseline": cpu, "parity": parity, "extra_configs": extras}
     if "parity_check" in parity:
         out["parity_check"] = parity["parity_check"]
+    if outputs is not None:
+        dump_outputs(outputs, args.dump_outputs)
     emit(out)
     if dist is not None:
         dist.destroy_process_group()

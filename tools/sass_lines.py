@@ -2,9 +2,11 @@
 lines by executed warp instructions.  Usage: sass_lines.py ncu_sass.csv nvdisasm.txt kernel_substring"""
 import collections
 import csv
+import os
 import re
 import sys
 
+CSRC = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "rmi_b200", "csrc")
 ncu_csv, dis_txt, kname = sys.argv[1:4]
 rows = list(csv.reader(open(ncu_csv)))
 hi = next(i for i, r in enumerate(rows) if "Source" in r and "Instructions Executed" in r)
@@ -44,7 +46,7 @@ srcs = {}
 for (f, ln), c in agg.most_common(40):
     if f not in srcs:
         try:
-            srcs[f] = open("/root/repo/rmi_b200/csrc/" + f).read().split("\n")
+            srcs[f] = open(os.path.join(CSRC, f)).read().split("\n")
         except Exception:
             srcs[f] = []
     text = srcs[f][ln - 1].strip()[:100] if 0 < ln <= len(srcs[f]) else ""
