@@ -259,6 +259,33 @@ void rmi_shard_comm_destroy(rmi_shard_comm* c);
 int rmi_shard_set_partition(rmi_shard_build* b, const uint64_t* bases, int world, int rank);
 int rmi_shard_train(rmi_shard_build* b, rmi_shard_comm* c, uint32_t flags, rmi_result** out);
 
+/* ---- Batched lookups on the GPU --------------------------------------------------------------
+ * A trained RMI uploaded to one device answers batches of device-resident queries: the generated
+ * code's lookup(key, &err) (codegen.rs:612-718), and the exact lower_bound position in the key set.
+ * Query and output arrays are device memory; 16-byte aligned arrays (any CUDA allocation) take the
+ * vectorised path.  Calls are enqueued on `cuda_stream` (NULL = the legacy default stream) with no
+ * host synchronisation; one index may be queried from several host threads at once.  The calling
+ * thread's current device is restored before each call returns.  Lookups for `--bounded` RMIs
+ * (the spline search of codegen.rs:720) are not offered: rmi_result does not carry the knots. */
+typedef struct rmi_index rmi_index;
+/* Upload a trained RMI (any rmi_result that holds its leaf tables) to `device`.  The index owns device
+ * copies of everything it needs: the result may be freed afterwards.  key_type = the key type of the data
+ * set the RMI was trained on, and of the queries. */
+int rmi_index_create(const rmi_result* r, rmi_key_type key_type, int device, rmi_index** out);
+/* pos[i] = min(leaf_t(q_i), num_rmi_rows - 1) with t = min(N - 1, top(q_i)), err[i] = last_layer_max_l1s[t]
+ * (err may be NULL), for n queries. */
+int rmi_index_predict(const rmi_index* ix, const void* d_queries, uint64_t n, uint64_t* d_pos, uint64_t* d_err,
+                      void* cuda_stream);
+/* Exact lower_bound: out[i] = number of keys k of `keys` with !(k >= q_i)  (= np.searchsorted(keys, q, "left")
+ * for every non-NaN query; a NaN query gets n).  `keys` must have the index's key type and length num_rmi_rows.
+ * The search covers the window [pos - err, pos + err + 1) and gallops outward when the answer lies outside it.
+ * d_fallbacks (nullable, one device u64) is incremented once per query whose answer lay outside the window. */
+int rmi_index_lower_bound(const rmi_index* ix, const rmi_dataset* keys, const void* d_queries, uint64_t n,
+                          uint64_t* d_out, uint64_t* d_fallbacks, void* cuda_stream);
+/* Device memory the index holds (leaf records, radix table, histogram pivots). */
+uint64_t rmi_index_device_bytes(const rmi_index* ix);
+void rmi_index_destroy(rmi_index* ix);
+
 /* ---- `--bounded` support: rmi_lib::cache_fix (reference rmi_lib/src/cache_fix.rs:106-150) ----------
  * The error-bounded spline over key -> first-occurrence offset whose interpolation always lands in
  * the key's line (offset / line_size).  A greedy, strictly serial HOST scan (as in the reference;

@@ -88,6 +88,13 @@ def load_library():
                                      C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64]
         L.rmi_find_pareto_efficient_configs.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.c_uint64, C.c_uint32,
                                                         C.POINTER(_ConfigStats), C.c_uint64, C.POINTER(C.c_uint64)]
+        L.rmi_index_create.argtypes = [C.POINTER(_Result), C.c_int, C.c_int, C.POINTER(C.c_void_p)]
+        L.rmi_index_predict.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.rmi_index_lower_bound.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
+                                            C.c_void_p]
+        L.rmi_index_device_bytes.restype = C.c_uint64
+        L.rmi_index_device_bytes.argtypes = [C.c_void_p]
+        L.rmi_index_destroy.argtypes = [C.c_void_p]
         _lib = L
     return _lib
 
@@ -391,3 +398,101 @@ def result_from_pointer(res, model_spec: str) -> TrainedRMI:
             l1_counts=_arr(r.l1_counts, N, C.c_uint64, np.uint64, owner),
             could_not_replace=bool(r.could_not_replace), top_fit_exact=bool(r.top_fit_exact), _res=owner)
     return out
+
+
+class RMIIndex:
+    """A trained RMI resident on one GPU that answers batches of lookups (rmi_index_* in include/rmi_b200.h).
+
+    ``trained``: a TrainedRMI returned by train() or a ctypes ``_Result`` that holds the leaf tables.  The index keeps
+    device copies of everything it needs, so the result may be freed afterwards.  ``key_type``: the key type of the
+    data set the RMI was trained on and of the queries (default: that of ``keys``).  ``keys``: that data set as an
+    RMITrainingData on the same device; lower_bound needs it.
+
+    ``predict(q) -> (pos, err)`` is the generated code's ``lookup(key, &err)`` per query, and ``lower_bound(q)`` the
+    exact ``np.searchsorted(keys, q, "left")`` (NaN queries: len(keys)).  Both take a numpy array of the key dtype
+    (copied to the device and back; the call returns when the results are on the host, as uint64 arrays) or a
+    contiguous CUDA torch tensor of the key dtype on the index's device (no copy; the work is enqueued on torch's
+    current stream and the results are int64 CUDA tensors, exact because positions are below 2^63).
+    """
+
+    def __init__(self, trained, key_type: int | None = None, device: int = 0, keys: RMITrainingData | None = None):
+        if key_type is None:
+            if keys is None:
+                raise ValueError("RMIIndex: key_type is required when no keys are given")
+            key_type = keys.key_type
+        self.key_type, self.device, self.keys = int(key_type), int(device), keys
+        self._h = C.c_void_p()
+        _check(load_library().rmi_index_create(_result_ptr(trained), self.key_type, self.device, C.byref(self._h)))
+
+    @property
+    def device_bytes(self) -> int:
+        """Device memory held by the index (leaf records, radix table, histogram pivots)."""
+        return int(load_library().rmi_index_device_bytes(self._live()))
+
+    def predict(self, q):
+        """(pos, err) per query."""
+        h = self._live()
+        return self._run(q, 2, lambda dq, n, outs, st: load_library().rmi_index_predict(h, dq, n, outs[0], outs[1], st))
+
+    def lower_bound(self, q, return_fallbacks: bool = False):
+        """Exact lower_bound per query.  With return_fallbacks, also the number of queries whose answer lay outside
+        the error window [pos - err, pos + err + 1) (an int on the numpy path, a one-element int64 tensor on the
+        torch path)."""
+        h = self._live()
+        if self.keys is None:
+            raise RMIError("RMIIndex.lower_bound needs the key set: pass keys= when creating the index")
+        ks = self.keys._h
+        out, fb = self._run(q, 1, lambda dq, n, outs, st: load_library().rmi_index_lower_bound(h, ks, dq, n, outs[0],
+                                                                                              outs[1], st),
+                            counter=True)
+        return (out, fb) if return_fallbacks else out
+
+    def close(self):
+        if getattr(self, "_h", None) and self._h.value:
+            load_library().rmi_index_destroy(self._h)
+            self._h = C.c_void_p()
+        self.keys = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    # -- plumbing --------------------------------------------------------------------------------------------------
+    def _live(self):
+        if not getattr(self, "_h", None) or not self._h.value:
+            raise RMIError("this RMIIndex is closed")
+        return self._h
+
+    def _run(self, q, n_out, call, counter=False):
+        """Run call(d_queries, n, [d_out...], stream) on device buffers; handles the numpy and the torch path."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        tdt = {KEY_U64: torch.uint64, KEY_U32: torch.uint32, KEY_F64: torch.float64}[self.key_type]
+        if isinstance(q, torch.Tensor):
+            if q.device != dev or q.dtype != tdt or not q.is_contiguous():
+                raise TypeError(f"RMIIndex: queries must be a contiguous {tdt} tensor on {dev} (got {q.dtype} on {q.device})")
+            dq, host = q, False
+        else:
+            qa = np.ascontiguousarray(q)
+            if qa.dtype != np.dtype(_NP_OF_KEY[self.key_type]):
+                raise TypeError(f"RMIIndex: queries must be {np.dtype(_NP_OF_KEY[self.key_type])} (got {qa.dtype})")
+            qa = qa.reshape(-1)
+            # signed views for the transfer: the bytes are what matters
+            dq = torch.from_numpy(qa.view({8: np.int64, 4: np.int32}[qa.itemsize])).to(dev)
+            host = True
+        n = dq.numel()
+        outs = [torch.empty(n, dtype=torch.int64, device=dev) for _ in range(n_out)]
+        fb = torch.zeros(1, dtype=torch.int64, device=dev) if counter else None
+        ptrs = [o.data_ptr() for o in outs] + ([fb.data_ptr()] if counter else [])
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _check(call(dq.data_ptr() if n else None, n, ptrs, stream))
+        if host:
+            res = [o.cpu().numpy().view(np.uint64) for o in outs]
+            if counter:
+                return res[0], int(fb.item())
+            return tuple(res) if n_out > 1 else res[0]
+        if counter:
+            return outs[0], fb
+        return tuple(outs) if n_out > 1 else outs[0]

@@ -15,7 +15,7 @@ _TAG = os.environ.get("RMI_BUILD_TAG", "")
 LIB_PATH = os.path.join(LIB_DIR, f"librmi_b200{'_' + _TAG if _TAG else ''}.so")
 OBJ_DIR = os.path.join(HERE, "build" + ("_" + _TAG if _TAG else ""))
 
-SOURCES = ["kernels_top.cu", "kernels_leaf.cu", "kernels_shard.cu", "api.cu"]
+SOURCES = ["kernels_top.cu", "kernels_leaf.cu", "kernels_shard.cu", "kernels_lookup.cu", "api.cu"]
 HEADERS = ["rust_math.cuh", "models.cuh", "device_util.cuh", "spline.cuh", "kernels.h",
            os.path.join("..", "..", "include", "rmi_b200.h"), os.path.join("..", "..", "host", "cache_fix.hpp"), os.path.join("..", "..", "host", "codegen.hpp"),
            os.path.join("..", "..", "host", "optimizer.hpp")]

@@ -453,6 +453,175 @@ void rmi_result_free(rmi_result* r) { delete reinterpret_cast<ResultBox*>(r); }
 
 }  // extern "C"
 
+// ---- batched lookups on a trained RMI (kernels_lookup.cu) ------------------------------------
+struct rmi_index {
+  int device = 0;
+  int key_type = 0;
+  LookupModel m{};         // device pointers below
+  void* d_leaves = nullptr;
+  u32* d_t32 = nullptr;
+  u64* d_pivots = nullptr;
+  uint64_t bytes = 0;
+};
+
+namespace {
+// Makes `device` current and gives the caller back its own device afterwards: lookups are enqueued
+// from threads that may be working on another GPU (torch code, for one, keeps a current device).
+struct DeviceScope {
+  int prev = -1;
+  cudaError_t err;
+  explicit DeviceScope(int device) {
+    if (cudaGetDevice(&prev) != cudaSuccess) prev = -1;
+    err = (prev == device) ? cudaSuccess : cudaSetDevice(device);
+  }
+  ~DeviceScope() { if (prev >= 0) cudaSetDevice(prev); }
+};
+
+void index_release(rmi_index* ix) {
+  cudaFree(ix->d_leaves);
+  cudaFree(ix->d_t32);
+  cudaFree(ix->d_pivots);
+  delete ix;
+}
+
+// Every argument check of rmi_index_create; no CUDA call.
+int index_check(const rmi_result* r, int key_type, rmi_index** out) {
+  if (!r || !out) return fail(RMI_ERR_INVALID, "rmi_index_create: null argument");
+  if (key_type < 0 || key_type > 2) return fail(RMI_ERR_INVALID, "rmi_index_create: bad key type " + std::to_string(key_type));
+  if (!r->l1_params || !r->l1_errors)
+    return fail(RMI_ERR_INVALID, "rmi_index_create: the result holds no leaf tables (built with RMI_FLAG_STATS_ONLY)");
+  if (r->l0_model_id > (uint32_t)M_HISTOGRAM)
+    return fail(RMI_ERR_INVALID, "rmi_index_create: unknown top model id " + std::to_string(r->l0_model_id));
+  if (r->l1_model_id > (uint32_t)M_LOGNORMAL)
+    return fail(RMI_ERR_INVALID, "rmi_index_create: unknown leaf model id " + std::to_string(r->l1_model_id));
+  if (r->l1_params_per_model != (uint32_t)leaf_params_per_model((int)r->l1_model_id))
+    return fail(RMI_ERR_INVALID, "rmi_index_create: l1_params_per_model does not match the leaf model");
+  if (r->branching_factor == 0 || r->num_rmi_rows == 0)
+    return fail(RMI_ERR_INVALID, "rmi_index_create: empty model (branching_factor or num_rmi_rows is 0)");
+  if (r->l0_model_id == (uint32_t)M_RADIX_TABLE) {
+    const uint32_t bits = r->l0_table_bits;
+    if (bits == 0 || bits > 32 || !r->l0_table32 || r->l0_table32_len != ((uint64_t)1 << bits))
+      return fail(RMI_ERR_INVALID, "rmi_index_create: a radix table top needs l0_table32 with 2^l0_table_bits entries");
+    // radix.rs:123-132 indexes the table with the key's bits after the common prefix; a prefix of 64
+    // (one distinct key) would shift by 0 and index past the table
+    if (r->l0_iparams[0] >= 64) return fail(RMI_ERR_INVALID, "rmi_index_create: radix table prefix must be below 64");
+  }
+  if (r->l0_model_id == (uint32_t)M_HISTOGRAM && r->l0_array2_len && !r->l0_array2)
+    return fail(RMI_ERR_INVALID, "rmi_index_create: histogram top without its pivots (l0_array2)");
+  return RMI_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int rmi_index_create(const rmi_result* r, rmi_key_type key_type, int device, rmi_index** out) {
+  if (int rc = index_check(r, (int)key_type, out)) return rc;
+  DeviceScope scope(device);
+  if (scope.err != cudaSuccess) return fail(RMI_ERR_CUDA, std::string("rmi_index_create: ") + cudaGetErrorString(scope.err));
+  auto* ix = new rmi_index();
+  ix->device = device;
+  ix->key_type = (int)key_type;
+  const uint64_t N = r->branching_factor;
+  const int leaf = (int)r->l1_model_id;
+  const size_t leaf_bytes = (size_t)N * lookup_record_words(leaf) * sizeof(u64);
+  std::vector<u64> packed((size_t)N * lookup_record_words(leaf));
+  lookup_pack_leaves(leaf, r->l1_params, reinterpret_cast<const u64*>(r->l1_errors), N, packed.data());
+  cudaError_t e = cudaMalloc(&ix->d_leaves, leaf_bytes);
+  if (e == cudaSuccess) e = cudaMemcpy(ix->d_leaves, packed.data(), leaf_bytes, cudaMemcpyHostToDevice);
+  ix->bytes = leaf_bytes;
+  TopModel& t = ix->m.top;
+  memset(&t, 0, sizeof(t));
+  t.kind = (int)r->l0_model_id;
+  t.high = r->l0_bradix_high ? 1 : 0;
+  t.table_bits = (int)r->l0_table_bits;
+  for (int q = 0; q < 4; ++q) { t.f[q] = r->l0_fparams[q]; t.ip[q] = r->l0_iparams[q]; }
+  if (e == cudaSuccess && t.kind == M_RADIX_TABLE) {
+    const size_t b = sizeof(u32) * r->l0_table32_len;
+    e = cudaMalloc(&ix->d_t32, b);
+    if (e == cudaSuccess) e = cudaMemcpy(ix->d_t32, r->l0_table32, b, cudaMemcpyHostToDevice);
+    ix->bytes += b;
+  }
+  if (e == cudaSuccess && t.kind == M_HISTOGRAM && r->l0_array2_len) {
+    // the pivots are all the histogram's prediction reads (histogram.rs:57-61, models.cuh top_predict)
+    const size_t b = sizeof(u64) * r->l0_array2_len;
+    e = cudaMalloc(&ix->d_pivots, b);
+    if (e == cudaSuccess) e = cudaMemcpy(ix->d_pivots, r->l0_array2, b, cudaMemcpyHostToDevice);
+    ix->bytes += b;
+  }
+  if (e != cudaSuccess) {
+    index_release(ix);
+    return fail(RMI_ERR_CUDA, std::string("rmi_index_create: ") + cudaGetErrorString(e));
+  }
+  t.t32 = ix->d_t32;
+  t.pivots = ix->d_pivots;
+  t.npivots = t.kind == M_HISTOGRAM ? r->l0_array2_len : 0;
+  ix->m.leaf_kind = leaf;
+  ix->m.leaves = ix->d_leaves;
+  ix->m.N = N;
+  ix->m.num_rows = r->num_rmi_rows;
+  *out = ix;
+  return RMI_OK;
+}
+
+int rmi_index_predict(const rmi_index* ix, const void* d_queries, uint64_t n, uint64_t* d_pos, uint64_t* d_err,
+                      void* cuda_stream) {
+  if (!ix) return fail(RMI_ERR_INVALID, "rmi_index_predict: null index");
+  if (n == 0) return RMI_OK;
+  if (!d_queries || !d_pos) return fail(RMI_ERR_INVALID, "rmi_index_predict: null query or output pointer");
+  DeviceScope scope(ix->device);
+  if (scope.err != cudaSuccess) return fail(RMI_ERR_CUDA, std::string("rmi_index_predict: ") + cudaGetErrorString(scope.err));
+  DeviceInfo di;
+  if (int rc = device_info(ix->device, &di)) return rc;
+  Launch L{(cudaStream_t)cuda_stream, di.num_sms};
+  u64* pos = reinterpret_cast<u64*>(d_pos);
+  u64* err = reinterpret_cast<u64*>(d_err);
+  switch (ix->key_type) {
+    case RMI_KEY_U64: lookup_predict<u64>(L, ix->m, (const u64*)d_queries, n, pos, err); break;
+    case RMI_KEY_U32: lookup_predict<u32>(L, ix->m, (const u32*)d_queries, n, pos, err); break;
+    default: lookup_predict<double>(L, ix->m, (const double*)d_queries, n, pos, err); break;
+  }
+  CUDA_TRY(cudaGetLastError());
+  return RMI_OK;
+}
+
+int rmi_index_lower_bound(const rmi_index* ix, const rmi_dataset* keys, const void* d_queries, uint64_t n, uint64_t* d_out,
+                          uint64_t* d_fallbacks, void* cuda_stream) {
+  if (!ix || !keys) return fail(RMI_ERR_INVALID, "rmi_index_lower_bound: null index or key set");
+  if (keys->key_type != ix->key_type)
+    return fail(RMI_ERR_INVALID, "rmi_index_lower_bound: the key set's key type (" + std::to_string(keys->key_type) +
+                                     ") is not the index's (" + std::to_string(ix->key_type) + ")");
+  if (keys->n != ix->m.num_rows)
+    return fail(RMI_ERR_INVALID, "rmi_index_lower_bound: the key set has " + std::to_string(keys->n) +
+                                     " keys, the index was trained on " + std::to_string(ix->m.num_rows));
+  if (keys->device != ix->device) return fail(RMI_ERR_INVALID, "rmi_index_lower_bound: the key set lives on another device");
+  if (n == 0) return RMI_OK;
+  if (!d_queries || !d_out) return fail(RMI_ERR_INVALID, "rmi_index_lower_bound: null query or output pointer");
+  DeviceScope scope(ix->device);
+  if (scope.err != cudaSuccess) return fail(RMI_ERR_CUDA, std::string("rmi_index_lower_bound: ") + cudaGetErrorString(scope.err));
+  DeviceInfo di;
+  if (int rc = device_info(ix->device, &di)) return rc;
+  Launch L{(cudaStream_t)cuda_stream, di.num_sms};
+  u64* out = reinterpret_cast<u64*>(d_out);
+  u64* fb = reinterpret_cast<u64*>(d_fallbacks);
+  switch (ix->key_type) {
+    case RMI_KEY_U64: lookup_lower_bound<u64>(L, ix->m, (const u64*)keys->d_keys, (const u64*)d_queries, n, out, fb); break;
+    case RMI_KEY_U32: lookup_lower_bound<u32>(L, ix->m, (const u32*)keys->d_keys, (const u32*)d_queries, n, out, fb); break;
+    default: lookup_lower_bound<double>(L, ix->m, (const double*)keys->d_keys, (const double*)d_queries, n, out, fb); break;
+  }
+  CUDA_TRY(cudaGetLastError());
+  return RMI_OK;
+}
+
+uint64_t rmi_index_device_bytes(const rmi_index* ix) { return ix ? ix->bytes : 0; }
+
+void rmi_index_destroy(rmi_index* ix) {
+  if (!ix) return;
+  DeviceScope scope(ix->device);
+  index_release(ix);
+}
+
+}  // extern "C"
+
 namespace {
 
 // Streams / events of the sliced leaf launch (kernels.h: LeafCopyOut), created once per host

@@ -170,4 +170,25 @@ void shard_copy_status(const Launch& L, const BuildAux* d_aux, unsigned* d_out);
 // {status word, could_not_replace != 0} of this rank, for the cross-rank gather (two_layer.rs:199-203 warns if ANY leaf could not be replaced)
 void shard_copy_flags(const Launch& L, const BuildAux* d_aux, unsigned* d_out2);
 
+// ---- batched lookups on a trained RMI (kernels_lookup.cu) ------------------------------------
+// A device-resident index: the top model (t32 / pivots point at device copies) and N leaf records of
+// lookup_record_words(leaf_kind) u64 words each, {params..., error bound, zero padding}: 32 bytes (one
+// sector) for the 2- and 3-parameter leaves, 64 bytes for cubic.
+struct LookupModel {
+  TopModel top;
+  int leaf_kind;
+  const void* leaves;
+  u64 N;          // leaf models (branching factor)
+  u64 num_rows;   // keys the RMI was trained on (> 0)
+};
+__host__ __device__ constexpr int lookup_record_words(int leaf_kind) { return leaf_kind == M_CUBIC ? 8 : 4; }
+// Host: the result's N x ppm parameters and N error bounds as N records (out: N * lookup_record_words words).
+void lookup_pack_leaves(int leaf_kind, const double* params, const u64* errors, u64 N, u64* out);
+// pos[i], err[i] (err may be null) of the generated code's lookup for the n queries q (device memory).
+template <class T> void lookup_predict(const Launch& L, const LookupModel& M, const T* q, u64 n, u64* pos, u64* err);
+// out[i] = number of keys (M.num_rows of them) k with !(k >= q[i]); *fallbacks (nullable) += queries whose answer lay
+// outside the error window.
+template <class T>
+void lookup_lower_bound(const Launch& L, const LookupModel& M, const T* keys, const T* q, u64 n, u64* out, u64* fallbacks);
+
 }  // namespace rmi

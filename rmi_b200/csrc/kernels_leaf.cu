@@ -1089,16 +1089,8 @@ template <int LEAF> __device__ __forceinline__ bool set_constant(double* f, u64 
   return false;
 }
 
-// Model::predict_to_int (models/mod.rs:735-737) = max(0, floor(p)) as u64, then clamped to n
-// by error_between.  The float->int conversion with round-toward-minus-infinity saturates
-// like Rust's cast (negative -> 0, too large -> MAX); NaN must be mapped to 0 by hand.  With
-// 32-bit indices (n < 2^32 - 1) the conversion saturates at 2^32 - 1 >= n, which the clamp to n
-// makes equivalent.
-template <int LEAF> __device__ __forceinline__ u64 leaf_predict64(const double* f, double x) {
-  double p = predict_float<LEAF>(f, x);
-  u64 v = (u64)__double2ull_rd(p);
-  return p != p ? 0ull : v;
-}
+// leaf_predict64 (models.cuh) is the 64-bit form.  With 32-bit indices (n < 2^32 - 1) the
+// conversion saturates at 2^32 - 1 >= n, which the clamp to n makes equivalent.
 // NANCHECK: leaf parameters (hence predictions) can only be NaN for float keys or for the
 // normal / lognormal / loglinear leaves; integer keys with linear / spline / cubic leaves
 // always give finite parameters, so the select is compiled out there.

@@ -71,6 +71,17 @@ template <int KIND> __device__ __forceinline__ u64 predict_int_f(const double* f
   return f64_to_u64_sat(floor(predict_float<KIND>(f, x)));
 }
 
+// Leaf-model Model::predict_to_int (models/mod.rs:735-737) = max(0, floor(p)) as u64.  The
+// float->int conversion with round-toward-minus-infinity saturates like Rust's cast (negative
+// -> 0, too large -> MAX); NaN must be mapped to 0 by hand.  The training forward pass
+// (kernels_leaf.cu) and the batched lookups (kernels_lookup.cu) both evaluate leaves with it,
+// so a lookup of a training key repeats the arithmetic its error bound was measured on.
+template <int LEAF> __device__ __forceinline__ u64 leaf_predict64(const double* f, double x) {
+  double p = predict_float<LEAF>(f, x);
+  u64 v = (u64)__double2ull_rd(p);
+  return p != p ? 0ull : v;
+}
+
 // Top-model prediction on a key (unclamped model index).
 template <int KIND, class T> __device__ __forceinline__ u64 top_predict(const TopModel& m, T key) {
   if (KIND <= M_LOGNORMAL) {
